@@ -5,6 +5,8 @@
   python bench.py --impl reference --gpus N --steps K ...      # the reference's own CPU path on the host cores
                                                                # (unmodified reference modules from baseline/_ref;
                                                                #  oracle port when the staged copy is absent)
+  python bench.py ... --dump-outputs DIR                       # also write the images of the last timed step
+                                                               # (rank 0) as DIR/images.npy, float32, <= 64 MB
 
 Workloads = BASELINE.json configs (SURVEY.md §8d), per GPU; --config 2 (the one the metric is quoted on) is the
 default: 512x512, SeeCoder + SD-v1.5 UNet, 50 DDIM steps, CFG 2.0, batch 4, fp16, synthetic seeded weights/inputs.
@@ -62,7 +64,13 @@ def parse():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-gpu-reference", action="store_true")
     ap.add_argument("--no-graph", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the images of the last timed step as DIR/<name>.npy (float32) to compare two builds")
     a = ap.parse_args()
+    if a.steps < 1:
+        ap.error("--steps must be at least 1")
+    if a.dump_outputs and a.impl != "ours":
+        ap.error("--dump-outputs applies to the pfd_b200 path only (--impl ours)")
     cfg = dict(CONFIGS[a.config])
     if a.batch:
         cfg["batch"] = a.batch
@@ -435,6 +443,25 @@ def gemm_roofline_pass(net, cfg, cond, uncond, hint):
     return stats["flops"], max(t_full - t_nogemm, 1e-6), stats["n"], br
 
 
+DUMP_LIMIT_BYTES = 64 * 2 ** 20
+
+
+def dump_outputs(directory, arrays):
+    """Write each tensor as <directory>/<name>.npy in float32, at most DUMP_LIMIT_BYTES in all.  A tensor over its
+    share is replaced by the elements at a fixed seeded set of flat indices (sorted), the same in every run of the
+    same arguments, so two builds can be compared element for element.  Compare with a tolerance: two runs of the same
+    build on the same inputs differed by 1.7e-3 relative rms in the config-2 images (B200, 1000 W power limit)."""
+    import numpy as np
+    os.makedirs(directory, exist_ok=True)
+    share = (DUMP_LIMIT_BYTES - 4096 * len(arrays)) // len(arrays)      # 4096: room for each .npy header
+    for name, t in arrays.items():
+        a = t.detach().float().cpu().numpy()
+        if a.nbytes > share:
+            idx = np.unique(np.random.default_rng(0).integers(0, a.size, share // a.itemsize))
+            a = a.reshape(-1)[idx]
+        np.save(os.path.join(directory, name + ".npy"), a)
+
+
 def load_traffic():
     """DRAM traffic of the dominant kernel from the committed ncu --set full capture (profiles/r2_traffic.json:
     dram__bytes_read.sum + dram__bytes_write.sum per launch of the named shape, algorithmic bytes beside it)."""
@@ -519,6 +546,8 @@ def run_ours(args):
     launches = nv.launch_count() - n0
     ms = e0.elapsed_time(e1)
     clk = clocks.stop()
+    if args.dump_outputs and rank == 0:                                  # before later requests reuse the buffers
+        dump_outputs(args.dump_outputs, {"images": im})
     # ---- e2e: host buffers, H2D of the reference image and D2H of the decoded images every step
     sync_all()
     e2, e3 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
