@@ -37,7 +37,7 @@ enum {
   PFD_ACT_NONE = 0,
   PFD_ACT_SILU = 1,   /* x*sigmoid(x)          (openaimodel.py:203 nn.SiLU, autokl_modules.py:33) */
   PFD_ACT_GELU = 2,   /* exact erf GELU        (swin.py:84 nn.GELU)                               */
-  PFD_ACT_RELU = 3,   /* seecoder.py:24 F.relu                                                    */
+  PFD_ACT_RELU = 3,   /* F.relu, NaN kept (seecoder.py:24, controlnet_annotator/hed/__init__.py:37) */
   PFD_ACT_GEGLU = 4   /* value*gelu(gate), weights packed [value|gate] per N tile (attention.py:44-51) */
 };
 
@@ -251,6 +251,35 @@ PFD_API int pfd_canny_f32(const void* x, int32_t src_is_f32, int32_t B, int32_t 
                           int32_t high, void* workspace, float* out, int32_t* sweeps_out, void* stream);
 /* ToTensor(ToPILImage(x)) = floor(x*255)/255 as float32 (controlnet.py:345-348, preprocess type 'input'). */
 PFD_API int pfd_image_u8_roundtrip_f32(const void* x, int32_t src_is_f32, int64_t n, float* out, void* stream);
+
+/*
+ * ControlNet.preprocess(type='hed' / 'softedge_v11p') on the GPU (controlnet.py:370-376 ->
+ * controlnet_annotator/hed/__init__.py:102-128).  The network's 3x3 convs (+ ReLU) run on pfd_gemm_f16 with every
+ * conv bias multiplied by a power-of-two activation scale s (ReLU and max-pool commute with it, so every activation
+ * is exactly s times the reference's; s keeps the raw 0-255 input's activations inside fp16).  Stream-ordered and
+ * capturable.
+ */
+#define PFD_HED_MAPS 5
+/* Network input (hed/__init__.py:111-113,52): x NCHW [B,3,H,W] fp16/fp32 in [0,1], quantised like ToPILImage,
+ * out[n,y,x,c] = fp16((u8 - norm[c]) * scale), channel-last [B,H,W,3].  norm: device fp32 [3].  The subtraction comes
+ * before the first conv's zero padding, as in the reference. */
+PFD_API int pfd_hed_input_f16(const void* x, int32_t src_is_f32, int32_t B, int32_t H, int32_t W, const float* norm,
+                              float scale, void* out, void* stream);
+/* 2x2 / stride-2 max-pool, channel-last [NB,H,W,C] -> [NB,H/2,W/2,C] (floor; hed/__init__.py:34 F.max_pool2d).
+ * C % 8 == 0. */
+PFD_API int pfd_maxpool2x2_f16(const void* x, int32_t NB, int32_t H, int32_t W, int32_t C, void* out, void* stream);
+/* 1x1 conv to one channel (DoubleConvBlock.projection, hed/__init__.py:30,38) with fp32 accumulation and output:
+ * out[m] = dot(x[m,:], w) * inv_scale + b[0] for channel-last fp16 x [M,C]; w device fp32 [C], b device fp32 [1].
+ * inv_scale = 1/s undoes the activation scale.  C % 8 == 0. */
+PFD_API int pfd_hed_project_f32(const void* x, int64_t M, int32_t C, const float* w, const float* b, float inv_scale,
+                                float* out, void* stream);
+/* The host tail of apply_hed (hed/__init__.py:118-128) + ToTensor / repeat (controlnet.py:373-375):
+ * maps[k] is a device fp32 [B, map_h[k], map_w[k]] logit map (host arrays of PFD_HED_MAPS entries, each map no
+ * larger than HxW); each is resized to HxW like cv2.resize(INTER_LINEAR) on float32, the maps are averaged in fp32,
+ * e = sigmoid(mean) in fp64, u8 = (uint8)clip(e*255, 0, 255); out float32 [B,3,H,W] = u8/255 in all three channels.
+ * *nonfinite (device int32, zeroed by the call) counts pixels whose mean logit is not finite. */
+PFD_API int pfd_hed_fuse_f32(const float* const* maps, const int32_t* map_h, const int32_t* map_w, int32_t B,
+                             int32_t H, int32_t W, float* out, int32_t* nonfinite, void* stream);
 
 #ifdef __cplusplus
 }

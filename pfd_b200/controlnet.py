@@ -5,7 +5,8 @@ Same constructor arguments / state-dict keys as the reference (spatial-transform
 ``UNetModel2D_Next.apply(control=...)``.  The hint stem (controlnet.py:165-181) depends only on the
 control image, so its output is cached per hint tensor instead of being recomputed every DDIM step.
 ``preprocess`` provides the annotator-free types on the GPU ('input', 'canny' — bit-exact cv2.Canny,
-SURVEY.md §8 f1); annotators that are networks of their own (controlnet.py:361-503) are outside the path.
+SURVEY.md §8 f1) and the HED soft-edge network ('hed', pfd_b200/hed.py); the other annotator networks
+(controlnet.py:361-503) are outside the path.
 """
 from __future__ import annotations
 
@@ -163,11 +164,12 @@ class ControlNet(nn.Module):
 
     @torch.no_grad()
     def preprocess(self, x, type="canny", **kwargs):
-        """controlnet.py:332-360 for the annotator-free types: 'none', 'input' / 'shuffle_v11e' (the uint8 round
-        trip of ToPILImage -> ToTensor) and 'canny' / 'canny_v11p' (cv2.Canny(rgb_u8, low, high), reproduced
-        bit-exactly on the GPU by pfd_canny_f32).  x: [B,3,H,W] tensor in [0,1] or an image path.  Returns float32
-        [B,3,H,W] on x's device.  Annotators that are networks of their own (midas, hed, mlsd, openpose, ...) are
-        outside the hot path (SURVEY.md §8 f1 names Canny only)."""
+        """controlnet.py:332-376 on the GPU for the types: 'none', 'input' / 'shuffle_v11e' (the uint8 round
+        trip of ToPILImage -> ToTensor), 'canny' / 'canny_v11p' (cv2.Canny(rgb_u8, low, high), reproduced
+        bit-exactly by pfd_canny_f32) and 'hed' / 'softedge_v11p' (the HED soft-edge network, pfd_b200.hed; its
+        weights ControlNetHED.pth are read from the reference's locations or set with pfd_b200.hed.set_network;
+        images must be at least 16x16).  x: [B,3,H,W] tensor in [0,1] or an image path.  Returns float32
+        [B,3,H,W] on x's device.  The other annotators (midas, mlsd, openpose, ...) raise NotImplementedError."""
         if type == "none" or type is None:
             return None
         if isinstance(x, str):
@@ -190,6 +192,9 @@ class ControlNet(nn.Module):
             high = kwargs.pop("high_threshold", 200)
             out, _ = nv.canny(x, int(low), int(high))
             return out
+        if type in ("hed", "softedge_v11p"):
+            from . import hed
+            return hed.run(x)
         raise NotImplementedError(f"controlnet annotator '{type}' is a separate network outside the pfd_b200 "
                                   "hot path; feed a ready control map (do_preprocess=False)")
 

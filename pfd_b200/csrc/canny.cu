@@ -18,26 +18,13 @@
 
 #include "../../include/pfd_b200.h"
 #include "common.h"
+#include "image_u8.cuh"
 
 namespace pfd {
 
 __device__ __forceinline__ void pdl_enter_c() {
   asm volatile("griddepcontrol.wait;" ::: "memory");
   asm volatile("griddepcontrol.launch_dependents;" ::: "memory");
-}
-
-// ToPILImage on a float tensor: pic.mul(255).byte() - the product is rounded in the tensor's dtype, then truncated
-template <typename T>
-__device__ __forceinline__ uint32_t to_u8(T v);
-template <>
-__device__ __forceinline__ uint32_t to_u8<float>(float v) {
-  const float m = v * 255.f;
-  return (uint32_t)(unsigned char)(int)m;
-}
-template <>
-__device__ __forceinline__ uint32_t to_u8<__half>(__half v) {
-  const float m = __half2float(__hmul(v, __float2half_rn(255.f)));
-  return (uint32_t)(unsigned char)(int)m;
 }
 
 template <typename T>

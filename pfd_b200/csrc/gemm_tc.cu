@@ -115,10 +115,18 @@ __device__ __forceinline__ float gelu_sig(float x) {
   return __fdividef(x, 1.f + e);
 }
 
+// max(v, 0) that keeps NaN, as F.relu does: an fp16 overflow upstream (inf - inf = NaN) must reach the output
+// instead of being flushed to 0
+__device__ __forceinline__ float relu_nan(float v) {
+  float r;
+  asm("max.NaN.f32 %0, %1, 0f00000000;" : "=f"(r) : "f"(v));
+  return r;
+}
+
 __device__ __forceinline__ float act_apply(float v, int act) {
   if (act == PFD_ACT_SILU) return __fdividef(v, 1.f + __expf(-v));
   if (act == PFD_ACT_GELU) return 0.5f * v * (1.f + fast_erf(v * 0.70710678118654752f));
-  if (act == PFD_ACT_RELU) return fmaxf(v, 0.f);
+  if (act == PFD_ACT_RELU) return relu_nan(v);
   return v;
 }
 

@@ -29,8 +29,10 @@ EXPORTS = [
     "pfd_add_rowvec_f16", "pfd_ddim_step_f16", "pfd_window_gather_f16", "pfd_window_scatter_f16",
     "pfd_patch_merge_gather_f16", "pfd_patchify_f16", "pfd_flash_attn_f16",
     "pfd_flash_attn_strided_f16", "pfd_ddim_begin_step", "pfd_vae_posterior_f16",
-    "pfd_canny_workspace_bytes", "pfd_canny_f32", "pfd_image_u8_roundtrip_f32",
+    "pfd_canny_workspace_bytes", "pfd_canny_f32", "pfd_image_u8_roundtrip_f32", "pfd_hed_input_f16",
+    "pfd_maxpool2x2_f16", "pfd_hed_project_f32", "pfd_hed_fuse_f32",
 ]
+PFD_HED_MAPS = 5
 
 
 class GemmDesc(ctypes.Structure):
@@ -125,6 +127,12 @@ def load() -> ctypes.CDLL:
     lib.pfd_canny_f32.argtypes = [c_void_p, c_int32, c_int32, c_int32, c_int32, c_int32, c_int32, c_void_p, c_void_p,
                                   POINTER(c_int32), c_void_p]
     lib.pfd_image_u8_roundtrip_f32.argtypes = [c_void_p, c_int32, c_int64, c_void_p, c_void_p]
+    lib.pfd_hed_input_f16.argtypes = [c_void_p, c_int32, c_int32, c_int32, c_int32, c_void_p, c_float, c_void_p,
+                                      c_void_p]
+    lib.pfd_maxpool2x2_f16.argtypes = [c_void_p, c_int32, c_int32, c_int32, c_int32, c_void_p, c_void_p]
+    lib.pfd_hed_project_f32.argtypes = [c_void_p, c_int64, c_int32, c_void_p, c_void_p, c_float, c_void_p, c_void_p]
+    lib.pfd_hed_fuse_f32.argtypes = [POINTER(c_void_p), POINTER(c_int32), POINTER(c_int32), c_int32, c_int32, c_int32,
+                                     c_void_p, c_void_p, c_void_p]
     for name in EXPORTS:
         if hasattr(lib, name) and name not in ("pfd_version", "pfd_last_error", "pfd_launch_count",
                                                "pfd_canny_workspace_bytes"):
@@ -500,6 +508,67 @@ def image_u8_roundtrip(x: torch.Tensor) -> torch.Tensor:
     _check(load().pfd_image_u8_roundtrip_f32(x.data_ptr(), int(x.dtype == torch.float32), x.numel(), out.data_ptr(),
                                              stream_ptr()), "pfd_image_u8_roundtrip_f32")
     return out
+
+
+def hed_input(x: torch.Tensor, norm: torch.Tensor, scale: float) -> torch.Tensor:
+    """NCHW [B,3,H,W] image in [0,1] (fp16/fp32) -> channel-last fp16 [B,H,W,3] = (floor(x*255) - norm[c]) * scale
+    (pfd_hed_input_f16); norm: CUDA fp32 [3]."""
+    if x.dim() != 4 or x.shape[1] != 3 or not x.is_cuda or x.dtype not in (torch.float16, torch.float32):
+        raise RuntimeError(f"hed_input: expected a CUDA fp16/fp32 [B,3,H,W] image, got {tuple(x.shape)} {x.dtype} {x.device}")
+    if norm.dtype != torch.float32 or norm.numel() != 3 or not norm.is_cuda:
+        raise RuntimeError("hed_input: norm must be a CUDA fp32 tensor of 3 values")
+    x, norm = x.contiguous(), norm.contiguous()
+    B, _, H, W = x.shape
+    out = torch.empty((B, H, W, 3), device=x.device, dtype=torch.float16)
+    _check(load().pfd_hed_input_f16(x.data_ptr(), int(x.dtype == torch.float32), B, H, W, norm.data_ptr(),
+                                    float(scale), out.data_ptr(), stream_ptr()), "pfd_hed_input_f16")
+    return out
+
+
+def maxpool2x2(x: torch.Tensor) -> torch.Tensor:
+    """2x2 / stride-2 max-pool (floor) of channel-last fp16 [NB,H,W,C] -> [NB,H/2,W/2,C] (pfd_maxpool2x2_f16)."""
+    _chk16(x, "maxpool2x2")
+    x = x.contiguous()
+    NB, H, W, C = x.shape
+    out = torch.empty((NB, H // 2, W // 2, C), device=x.device, dtype=torch.float16)
+    _check(load().pfd_maxpool2x2_f16(x.data_ptr(), NB, H, W, C, out.data_ptr(), stream_ptr()), "pfd_maxpool2x2_f16")
+    return out
+
+
+def hed_project(x: torch.Tensor, w: torch.Tensor, b: torch.Tensor, inv_scale: float = 1.0) -> torch.Tensor:
+    """1x1 conv to one channel with fp32 accumulation: channel-last fp16 [NB,H,W,C] -> fp32 [NB,H,W] =
+    dot(x, w) * inv_scale + b (pfd_hed_project_f32); w: CUDA fp32 [C], b: CUDA fp32 [1]."""
+    _chk16(x, "hed_project")
+    x = x.contiguous()
+    NB, H, W, C = x.shape
+    if w.dtype != torch.float32 or b.dtype != torch.float32 or w.numel() != C or b.numel() != 1 or not w.is_cuda \
+            or not b.is_cuda:
+        raise RuntimeError(f"hed_project: expected CUDA fp32 w [{C}] and b [1]")
+    out = torch.empty((NB, H, W), device=x.device, dtype=torch.float32)
+    _check(load().pfd_hed_project_f32(x.data_ptr(), NB * H * W, C, w.contiguous().data_ptr(), b.data_ptr(),
+                                      float(inv_scale), out.data_ptr(), stream_ptr()), "pfd_hed_project_f32")
+    return out
+
+
+def hed_fuse(maps: Sequence[torch.Tensor], H: int, W: int,
+             nonfinite: Optional[torch.Tensor] = None) -> Tuple[torch.Tensor, torch.Tensor]:
+    """Five fp32 logit maps [B,h_k,w_k] -> (float32 [B,3,H,W] edge map, CUDA int32 [1] count of non-finite mean
+    logits) (pfd_hed_fuse_f32: cv2 INTER_LINEAR resize, mean, sigmoid, uint8 truncation)."""
+    if len(maps) != PFD_HED_MAPS:
+        raise RuntimeError(f"hed_fuse: expected {PFD_HED_MAPS} maps, got {len(maps)}")
+    B = maps[0].shape[0]
+    for m in maps:
+        if m.dtype != torch.float32 or m.dim() != 3 or m.shape[0] != B or not m.is_cuda or not m.is_contiguous():
+            raise RuntimeError(f"hed_fuse: expected contiguous CUDA fp32 [B,h,w] maps, got {tuple(m.shape)} {m.dtype}")
+    out = torch.empty((B, 3, H, W), device=maps[0].device, dtype=torch.float32)
+    if nonfinite is None:
+        nonfinite = torch.empty(1, device=maps[0].device, dtype=torch.int32)
+    ptrs = (c_void_p * PFD_HED_MAPS)(*[m.data_ptr() for m in maps])
+    hs = (c_int32 * PFD_HED_MAPS)(*[m.shape[1] for m in maps])
+    ws = (c_int32 * PFD_HED_MAPS)(*[m.shape[2] for m in maps])
+    _check(load().pfd_hed_fuse_f32(ptrs, hs, ws, B, H, W, out.data_ptr(), nonfinite.data_ptr(), stream_ptr()),
+           "pfd_hed_fuse_f32")
+    return out, nonfinite
 
 
 def window_gather(x: torch.Tensor, ws: int, shift: int) -> torch.Tensor:
